@@ -72,7 +72,36 @@ def parse():
                     help="chain workload: copy the revolutions out of the node stream (rpl_assemble_scans_dev) instead of "
                          "handing views to the scan kernel")
     ap.add_argument("--no-cloud", action="store_true", help="skip the PointCloud2 + exchange leg (extra.cloud)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="scan workload: after the timed steps, write what the last one returned (rank 0) as "
+                         "DIR/<name>.npy, float32 or float64, for a fixed seeded sample of the scans")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "scan"):
+        ap.error("--dump-outputs writes the outputs of the scan workload of this repo's path")
+    return args
+
+
+DUMP_BYTES = 60 << 20  # what --dump-outputs writes stays under 64 MB
+
+
+def dump_scan_outputs(out_dir, ranges, intens, beams, inc, status):
+    """The LaserScans of a fixed seeded sample of the batch, as a caller of rpl_scan_batch_dev receives them:
+    ranges and intensities [k, nodes] (zero past each scan's beam count, where nothing is written), and per scan
+    the beam count, angle increment and ascendScanData status.  scan_index holds the sampled scans' indices."""
+    S, N = ranges.shape
+    k = max(1, min(S, DUMP_BYTES // (8 * N + 32)))
+    idx = np.sort(np.random.default_rng(0).choice(S, k, replace=False))
+    sel = lambda t: t[idx].cpu().numpy()  # noqa: E731
+    b = sel(beams)
+    past = np.arange(N)[None, :] >= b[:, None]
+    arrays = {"scan_index": idx.astype(np.float64), "beam_counts": b.astype(np.float64),
+              "angle_increment": sel(inc).astype(np.float32), "status": sel(status).view(np.uint32).astype(np.float64),
+              "ranges": np.where(past, np.float32(0), sel(ranges)), "intensities": np.where(past, np.float32(0), sel(intens))}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def workload_name(args):
@@ -466,6 +495,8 @@ def run_b200(args, rank, local_rank, world):
     params = R.scan_params(0, mode_a, 0, 1)
     ms, prof, launches, win = timed(params, args.steps, max(args.warmup, 3), profile=True)
     sampler.window(win[0], win[1], "timed region")
+    if args.dump_outputs and rank == 0:  # before the legs below reuse the buffers
+        dump_scan_outputs(args.dump_outputs, ranges, intens, beams, inc, status)
     pts_step = S * N
     value = world * pts_step * args.steps / (ms * 1e-3) / 1e6
     n_fast = int((path == 0).sum().item())

@@ -27,5 +27,15 @@ def oracle():
 
 
 @pytest.fixture(scope="session")
+def reference(oracle):
+    """The reference's outputs: live from oracle/_ref where it is built, else as stored digests."""
+    from reference_outputs import Reference
+
+    r = Reference(oracle)
+    yield r
+    r.save()
+
+
+@pytest.fixture(scope="session")
 def golden_dir():
     return os.path.join(ROOT, "tests", "golden")

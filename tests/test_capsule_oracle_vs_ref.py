@@ -1,18 +1,18 @@
 """SURVEY.md 8(f) rank 1, the other answer formats -- pins oracle/capsule_oracle.cpp against the SDK's
-OWN LIDARSampleDataUnpacker compiled in place (oracle/_ref): express (0x82), HQ (0x83), ultra (0x84)
-and ultra-dense (0x86) capsules and the 5-byte standard nodes (0x81), node for node and event for
-event, with random payload bits so that every field is exercised.  CPU only."""
+OWN LIDARSampleDataUnpacker compiled in place (oracle/_ref; its outputs are also stored as digests, see
+tests/reference_outputs.py): express (0x82), HQ (0x83), ultra (0x84) and ultra-dense (0x86) capsules and the
+5-byte standard nodes (0x81), node for node and event for event, with random payload bits so that every field is
+exercised.  CPU only."""
 import numpy as np
 import pytest
 
-from test_decode_oracle_vs_ref import expected_events
+from test_decode_oracle_vs_ref import expected_events, ref  # noqa: F401  (ref: the fixture)
 
 
-@pytest.fixture(scope="module")
-def ref(oracle):
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref not built (reference tree absent on this box)")
-    return oracle
+def unpacked_nodes(O, ans, stream, sample_us, chunk, ours):
+    """The nodes the SDK's unpacker makes of a raw byte stream must be `ours`."""
+    O.reference.check("unpacker nodes", (ans, stream, sample_us, chunk), (ours,),
+                      lambda: (O.ref_unpack(ans, stream, sample_us, chunk)[0],))
 
 
 def make_capsules(O, ans, n, caps_per_rev=60.0, seed=0, sync_every=None, near=False):
@@ -43,11 +43,8 @@ def make_capsules(O, ans, n, caps_per_rev=60.0, seed=0, sync_every=None, near=Fa
 
 def check(O, ans, caps, sample_us=31, chunk=0, state=(0, 0)):
     nodes, status, offs, out_state = O.decode_capsules(ans, caps, sample_us, state)
-    rnodes, revents = O.ref_unpack(ans, caps.reshape(-1), sample_us, chunk)
-    assert len(nodes) == len(rnodes)
-    assert (nodes.view(np.uint64) == rnodes.view(np.uint64)).all()
-    exp = expected_events(O, status, offs)
-    assert exp.shape == revents.shape and (exp == revents).all()
+    O.reference.check("unpacker", (ans, caps, sample_us, chunk, state), (nodes, expected_events(O, status, offs)),
+                      lambda: O.ref_unpack(ans, caps.reshape(-1), sample_us, chunk))
     return nodes, status
 
 
@@ -117,9 +114,8 @@ def test_standard_nodes_with_byte_level_resync(ref):
     rec[:, 3:] = rng.integers(0, 256, (n, 2))
     clean = rec.reshape(-1)
     nodes, ends, pos = O.decode_normal(clean)
-    rn, _ = O.ref_unpack(0x81, clean, 476, 0)
+    unpacked_nodes(O, 0x81, clean, 476, 0, nodes)
     assert len(nodes) == n and pos == 0 and (ends == np.arange(n) * 5 + 4).all()
-    assert (nodes.view(np.uint64) == rn.view(np.uint64)).all()
     # garbage: inserted / dropped / corrupted bytes make the state machine hunt for the next record
     for seed in range(8):
         r = np.random.default_rng(seed)
@@ -128,11 +124,9 @@ def test_standard_nodes_with_byte_level_resync(ref):
         b = np.delete(b, r.choice(len(b), 50, replace=False))
         b = np.insert(b, np.sort(r.choice(len(b), 50, replace=False)), r.integers(0, 256, 50).astype(np.uint8))
         nodes, _, _ = O.decode_normal(b)
-        rn, _ = O.ref_unpack(0x81, b, 476, int(r.integers(0, 9)))
-        assert len(nodes) == len(rn) and 0 < len(nodes) < n
-        assert (nodes.view(np.uint64) == rn.view(np.uint64)).all()
+        unpacked_nodes(O, 0x81, b, 476, int(r.integers(0, 9)), nodes)
+        assert 0 < len(nodes) < n
     # pure noise
     b = rng.integers(0, 256, 20000, dtype=np.uint8)
     nodes, _, _ = O.decode_normal(b)
-    rn, _ = O.ref_unpack(0x81, b, 476, 0)
-    assert len(nodes) == len(rn) and (nodes.view(np.uint64) == rn.view(np.uint64)).all()
+    unpacked_nodes(O, 0x81, b, 476, 0, nodes)

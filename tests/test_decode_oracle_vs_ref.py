@@ -1,15 +1,16 @@
 """SURVEY.md 8(f) rank 1 -- dense-capsule decode.  Pins the restatement (oracle/decode_oracle.cpp)
-against the SDK's OWN LIDARSampleDataUnpacker compiled in place (oracle/_ref): node for node and
-event for event (scan resets, checksum errors, encoder-reset errors), including byte streams fed
-in odd chunk sizes.  CPU only."""
+against the SDK's OWN LIDARSampleDataUnpacker compiled in place (oracle/_ref; its outputs are also stored as
+digests, see tests/reference_outputs.py): node for node and event for event (scan resets, checksum errors,
+encoder-reset errors), including byte streams fed in odd chunk sizes.  CPU only."""
 import numpy as np
 import pytest
 
 
 @pytest.fixture(scope="module")
-def ref(oracle):
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref not built (reference tree absent on this box)")
+def ref(oracle, reference):
+    # the helpers here and in the other *_vs_ref modules are handed the oracle module and reach the reference
+    # outputs through it
+    oracle.reference = reference
     return oracle
 
 
@@ -44,13 +45,10 @@ def expected_events(O, status, offs):
 
 
 def check(O, caps, sample_us=31, chunk=84):
-    nodes, status, offs, out_state = O.dense_decode(caps, sample_us, RefState.value)
-    rnodes, revents = O.ref_dense_decode(caps.reshape(-1), sample_us, chunk)
-    RefState.value = out_state
-    assert len(nodes) == len(rnodes)
-    assert (nodes.view(np.uint64) == rnodes.view(np.uint64)).all()
-    exp = expected_events(O, status, offs)
-    assert exp.shape == revents.shape and (exp == revents).all()
+    state = RefState.value
+    nodes, status, offs, RefState.value = O.dense_decode(caps, sample_us, state)
+    O.reference.check("dense capsule unpacker", (caps, sample_us, chunk, state), (nodes, expected_events(O, status, offs)),
+                      lambda: O.ref_dense_decode(caps.reshape(-1), sample_us, chunk))
     return nodes, status
 
 
@@ -112,16 +110,18 @@ def test_random_streams(ref):
 
 
 # ---- scan assembly (8(f) rank 2): restatement vs the reference's real ScanDataHolder ----------------
-def _same_scans(a, b):
-    (sa, la, ka), (sb, lb, kb) = a, b
-    assert ka == kb and (la == lb).all()
-    for k in range(min(ka, len(la))):
-        assert (sa[k, : la[k]].view(np.uint64) == sb[k, : lb[k]].view(np.uint64)).all(), k
+def _scans(res):
+    s, lens, k = res
+    return (k, lens) + tuple(s[i, : lens[i]] for i in range(min(k, len(lens))))
+
+
+def _same_scans(O, nodes, resets, max_nodes, max_scans):
+    O.reference.check("ScanDataHolder", (nodes, resets, max_nodes, max_scans),
+                      _scans(O.assemble_scans(nodes, resets, max_nodes, max_scans)),
+                      lambda: _scans(O.ref_assemble_scans(nodes, resets, max_nodes, max_scans)))
 
 
 def test_scan_assembly_matches_reference_holder(ref):
-    if not ref.have_ref_holder():
-        pytest.skip("oracle/_ref/libref_holder.so not built")
     rng = np.random.default_rng(3)
     for t in range(30):
         caps = make_stream(ref, int(rng.integers(50, 900)), float(rng.uniform(20, 200)), seed=500 + t,
@@ -129,7 +129,7 @@ def test_scan_assembly_matches_reference_holder(ref):
         nodes, status, offs, _ = ref.dense_decode(caps, 31, 0)
         resets = ref.resets_from_capsules(status, offs)
         for max_nodes in (8192, 500):
-            _same_scans(ref.assemble_scans(nodes, resets, max_nodes, 64), ref.ref_assemble_scans(nodes, resets, max_nodes, 64))
+            _same_scans(ref, nodes, resets, max_nodes, 64)
     # hand-made corner cases: nothing before the first scan start, resets at and between starts, cap
     mk = ref.make_nodes
     flags = np.array([2, 2, 1, 2, 2, 1, 2, 1, 1, 2, 2, 2, 1, 2], np.uint8)
@@ -137,4 +137,4 @@ def test_scan_assembly_matches_reference_holder(ref):
     for resets in ([], [0], [2], [3], [5], [6, 7], [8], [12], [13], [3, 9, 12]):
         r = np.array(resets, np.uint32)
         for max_nodes in (8192, 2, 1):
-            _same_scans(ref.assemble_scans(nodes, r, max_nodes, 16), ref.ref_assemble_scans(nodes, r, max_nodes, 16))
+            _same_scans(ref, nodes, r, max_nodes, 16)

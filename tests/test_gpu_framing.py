@@ -3,6 +3,8 @@ tests/test_framing_vs_ref.py pins against the SDK's own unpacker on damaged stre
 import numpy as np
 import pytest
 
+from test_capsule_oracle_vs_ref import unpacked_nodes
+from test_decode_oracle_vs_ref import ref  # noqa: F401  (the fixture)
 from test_framing_vs_ref import FORMATS, damaged_stream
 
 pytestmark = pytest.mark.gpu
@@ -68,13 +70,12 @@ def test_framer_matches_the_oracle_on_damaged_and_long_streams(R, oracle, ans):
 
 
 @pytest.mark.parametrize("ans", FORMATS)
-def test_raw_bytes_to_nodes_on_the_device_equals_the_sdk(R, oracle, ans):
+def test_raw_bytes_to_nodes_on_the_device_equals_the_sdk(R, ref, ans):
     """raw damaged bytes -> rpl_frame_capsules_dev -> rpl_decode_capsules_batch_dev, no host round trip, against the
     SDK's own unpacker fed the same bytes."""
     import torch
 
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref not built")
+    oracle = ref
     ctx = R.Context(0, 8192, 1)
     rng = np.random.default_rng(500 + ans)
     streams = [damaged_stream(oracle, ans, rng, ncap=300, max_edits=8) for _ in range(16)]
@@ -90,7 +91,5 @@ def test_raw_bytes_to_nodes_on_the_device_equals_the_sdk(R, oracle, ans):
     torch.cuda.synchronize()
     hn, hc = nodes.cpu().numpy(), ncount.cpu().numpy()
     for i, s in enumerate(streams):
-        rn, _ = oracle.ref_unpack(ans, s, 31)
-        assert hc[i] == len(rn), (hex(ans), i, hc[i], len(rn))
-        assert (hn[i, : hc[i]].view(np.uint64).reshape(-1) == rn.view(np.uint64)).all(), (hex(ans), i)
+        unpacked_nodes(oracle, ans, s, 31, 0, np.ascontiguousarray(hn[i, : hc[i]]).view(oracle.NODE_DTYPE).reshape(-1))
     ctx.close()

@@ -1,20 +1,20 @@
 """SURVEY.md 8(f) rank 4 -- per-sample timestamps.  Pins oracle/timestamp_oracle.cpp against the SDK's own
 unpackers running on a settable clock (oracle/_ref/libref_clock.so: the SDK compiled without its
-timer.cpp) and the scan-begin timestamp against the real ScanDataHolder.  CPU only."""
+timer.cpp) and the scan-begin timestamp against the real ScanDataHolder; their outputs are also stored as
+digests, see tests/reference_outputs.py.  CPU only."""
 import numpy as np
 import pytest
 
 from test_capsule_oracle_vs_ref import make_capsules
-from test_decode_oracle_vs_ref import make_stream
+from test_decode_oracle_vs_ref import make_stream, ref  # noqa: F401  (ref: the fixture)
 
 TIMINGS = [(31, 0, 0, 0), (63, 256000, 17, 0), (125, 1000000, 0, 2), (476, 115200, 250, 0), (31, 460800, 5, 1)]
 
 
-@pytest.fixture(scope="module")
-def ref(oracle):
-    if not (oracle.have_ref_clock() and oracle.have_ref_holder()):
-        pytest.skip("oracle/_ref not built (reference tree absent on this box)")
-    return oracle
+def timestamped_nodes(O, ans, stream, chunk, rx, t4, nodes, ts):
+    """The SDK's unpacker on its settable clock must give `nodes` stamped `ts`."""
+    O.reference.check("unpacker on a clock", (ans, stream, chunk, rx, t4), (nodes, ts),
+                      lambda: O.ref_unpack_ts(ans, stream, chunk, rx, t4))
 
 
 def rx_times(n, seed):
@@ -36,9 +36,8 @@ def test_capsule_node_timestamps(ref, ans, timing):
     rx = rx_times(n, ans)
     nodes, status, offs, _ = O.decode_capsules(ans, caps, timing[0])
     ts = O.node_timestamps(ans, t4, rx, status, offs, len(nodes))
-    rnodes, rts = O.ref_unpack_ts(ans, caps.reshape(-1), O.capsule_bytes(ans), rx, t4)
-    assert len(rnodes) == len(nodes) > 0
-    assert (rts == ts).all()
+    timestamped_nodes(O, ans, caps.reshape(-1), O.capsule_bytes(ans), rx, t4, nodes, ts)
+    assert len(nodes) > 0
 
 
 @pytest.mark.parametrize("timing", TIMINGS)
@@ -59,8 +58,8 @@ def test_standard_node_timestamps(ref, timing):
         rx = rx_times((len(b) + chunk - 1) // chunk, chunk)
         nodes, ends, _ = O.decode_normal(b)
         ts = O.normal_timestamps(t4, ends, chunk, rx)
-        rnodes, rts = O.ref_unpack_ts(0x81, b, chunk, rx, t4)
-        assert len(rnodes) == len(nodes) > 0 and (rts == ts).all()
+        timestamped_nodes(O, 0x81, b, chunk, rx, t4, nodes, ts)
+        assert len(nodes) > 0
 
 
 def test_scan_begin_timestamp_matches_the_reference_holder(ref):
@@ -72,8 +71,12 @@ def test_scan_begin_timestamp_matches_the_reference_holder(ref):
     ts = O.node_timestamps(0x85, t4, rx, status, offs, len(nodes))
     resets = O.resets_from_capsules(status, offs)
     e, elen, ek, ets = O.assemble_scans_ts(nodes, ts, resets, 8192, 16)
-    r, rlen, rk, rts = O.ref_assemble_scans_ts(nodes, ts, resets, 8192, 16)
-    assert ek == rk and ek >= 4
-    assert (elen[:ek] == rlen[:rk]).all() and (ets[:ek] == rts[:rk]).all()
+
+    def begins(scans, lens, k, sts):
+        return k, lens[:k], sts[:k]
+
+    O.reference.check("ScanDataHolder timestamps", (nodes, ts, resets, 8192, 16), begins(e, elen, ek, ets),
+                      lambda: begins(*O.ref_assemble_scans_ts(nodes, ts, resets, 8192, 16)))
+    assert ek >= 4
     starts = np.flatnonzero(nodes["flag"] & 1)
     assert set(ets[:ek].tolist()) <= set(ts[starts].tolist())
