@@ -189,7 +189,8 @@ rpl_result rpl_cloud_batch(rpl_ctx* ctx, const rpl_node_hq* nodes, const uint32_
                            float* xyzi, uint32_t* point_counts);
 /* Packs the per-scan clouds of a batch into one dense cloud (the per-GPU "fused cloud" that
  * is all-gathered across ranks): fused[0..*total) points, 16 B each; offsets[s] = first point
- * of scan s.  fused must hold n_scans*stride points. */
+ * of scan s.  fused must hold n_scans*stride points.  An empty batch (n_scans == 0) sets *total = 0, as do the push
+ * and the exchange below for the count they publish. */
 rpl_result rpl_cloud_fuse_dev(rpl_ctx* ctx, const float* xyzi, const uint32_t* point_counts,
                               uint32_t n_scans, uint32_t stride, float* fused, uint32_t* offsets,
                               uint32_t* total, void* stream);
@@ -409,7 +410,10 @@ rpl_result rpl_assemble_scan_views_starts_dev(rpl_ctx* ctx, rpl_node_hq* nodes, 
                                               uint64_t* scan_begin_ts_us, void* stream);
 /* rpl_scan_batch_dev over views: scan s = views[s].count nodes from nodes[views[s].first]; nodes_total = nodes in
  * the buffer; outputs laid out [n_scans][stride] as before (stride >= every count, stride <= 8192: the views are
- * served by the shared-memory kernels).  `nodes` must be 16-byte aligned. */
+ * served by the shared-memory kernels).  `nodes` must be 16-byte aligned.  A view with first + count > nodes_total
+ * is reported like a count above the stride: status[s] = RPL_RESULT_INVALID_DATA, beam count 0, nothing else written.
+ * nodes_out requires params->apply_ascend (RPL_RESULT_INVALID_DATA otherwise, nothing enqueued): without the ascend
+ * the unchanged nodes are the views themselves. */
 rpl_result rpl_scan_views_dev(rpl_ctx* ctx, const rpl_node_hq* nodes, uint64_t nodes_total, const rpl_scan_view* views,
                               uint32_t n_scans, uint32_t stride, const rpl_scan_params* params, rpl_node_hq* nodes_out,
                               float* ranges, float* intensities, uint32_t* beam_counts, float* angle_increment,
@@ -424,8 +428,9 @@ rpl_result rpl_scan_views_dev(rpl_ctx* ctx, const rpl_node_hq* nodes, uint64_t n
  * point cross the host link on the way in instead of the 8 of a decoded node.  capsules: host
  * [n_streams][stride_capsules][84]; outputs: host ranges / intensities [n_streams * max_scans][max_nodes],
  * beam_counts / angle_increment (nullable) [n_streams * max_scans] (slot k of stream s at s * max_scans + k; unused
- * slots have beam count 0), scans_per_stream [n_streams].  max_nodes: even, <= 8192, at least the longest
- * revolution (longer ones are cut by the holder's capacity rule); the context's max_scans must cover
+ * slots have beam count 0), scans_per_stream [n_streams].  max_nodes: even, <= 8192, at most the context's max_nodes
+ * (RPL_RESULT_INVALID_DATA otherwise), at least the longest revolution (longer ones are cut by the holder's capacity
+ * rule); the context's max_scans must cover
  * max_scans of at least one stream.  Pinned host memory (rpl_host_alloc) keeps the copies asynchronous. */
 rpl_result rpl_chain_dense_laserscan(rpl_ctx* ctx, const uint8_t* capsules, const uint32_t* capsule_counts,
                                      uint32_t n_streams, uint32_t stride_capsules, uint32_t sample_duration_us,

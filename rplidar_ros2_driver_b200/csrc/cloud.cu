@@ -394,9 +394,9 @@ cudaError_t launch_cloud_fuse_push(const float4* xyzi, const uint32_t* point_cou
                                    uint32_t stride, const PeerBases& peers, uint32_t world, uint32_t rank,
                                    uint32_t slot_points, uint32_t* offsets, uint32_t* total, cudaStream_t stream,
                                    int* launched) {
-  if (n_scans == 0) return cudaSuccess;
+  // an empty batch still runs both kernels: *total = 0 and the header entries must not keep an earlier step's count
   cloud_offsets_kernel<<<1, 1024, 0, stream>>>(point_counts, n_scans, offsets, total);
-  const uint32_t gy = min(n_scans, 65535u);
+  const uint32_t gy = max(1u, min(n_scans, 65535u));
   const uint32_t gx = max(1u, min(32u, (stride + 255u) / 256u));
   cloud_push_kernel<<<dim3(gx, gy), 256, 0, stream>>>(xyzi, point_counts, offsets, total, n_scans, stride, peers,
                                                       world, rank, slot_points);
@@ -478,9 +478,9 @@ cudaError_t launch_cloud_post(float4* xyzi, uint32_t* point_counts, uint32_t n_s
 cudaError_t launch_cloud_fuse(const float4* xyzi, const uint32_t* point_counts, uint32_t n_scans,
                               uint32_t stride, float4* fused, uint32_t capacity, uint32_t* offsets, uint32_t* total,
                               cudaStream_t stream, int* launched) {
-  if (n_scans == 0) return cudaSuccess;
+  // an empty batch still runs the offsets kernel: it writes *total = 0 (the caller's count, or a gather slot's header)
   cloud_offsets_kernel<<<1, 1024, 0, stream>>>(point_counts, n_scans, offsets, total);
-  const uint32_t gy = min(n_scans, 65535u);
+  const uint32_t gy = max(1u, min(n_scans, 65535u));
   const uint32_t gx = max(1u, min(32u, (stride + 255u) / 256u));
   cloud_pack_kernel<<<dim3(gx, gy), 256, 0, stream>>>(xyzi, point_counts, offsets, n_scans, stride, fused, capacity);
   if (launched) *launched += 2;

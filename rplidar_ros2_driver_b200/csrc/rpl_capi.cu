@@ -1168,6 +1168,11 @@ rpl_result rpl_scan_views_dev(rpl_ctx* c, const rpl_node_hq* nodes, uint64_t nod
     c->err = "the node buffer of a view batch must be 16-byte aligned";
     return RPL_RESULT_INVALID_DATA;
   }
+  if (nodes_out && !params->apply_ascend) {
+    // the batch path's pass-through is one strided copy of [n_scans][stride] nodes, which views do not have
+    c->err = "nodes_out of a view batch needs apply_ascend (the unascended nodes are the views themselves)";
+    return RPL_RESULT_INVALID_DATA;
+  }
   RPL_CUDA(c, cudaSetDevice(c->device), RPL_RESULT_OPERATION_FAIL);
   cudaStream_t st = stream ? static_cast<cudaStream_t>(stream) : c->lane[0].stream;
   return enqueue_scan(c, c->lane[0], nodes, reinterpret_cast<const uint32_t*>(views), n_scans, stride, params, nodes_out,
@@ -1186,6 +1191,11 @@ rpl_result rpl_chain_dense_laserscan(rpl_ctx* c, const uint8_t* capsules, const 
   if (n_streams == 0) return RPL_RESULT_OK;
   if (max_nodes == 0 || max_nodes > rpl::kSmallMaxNodes || (max_nodes & 1u) || max_scans == 0 || stride_capsules == 0) {
     c->err = "need an even max_nodes in [2, 8192] (the longest revolution), max_scans > 0, stride_capsules > 0";
+    return RPL_RESULT_INVALID_DATA;
+  }
+  if (max_nodes > c->max_nodes) {
+    // the scan kernels would report every longer revolution as INVALID_DATA into a status nobody reads
+    c->err = "max_nodes exceeds the context's max_nodes";
     return RPL_RESULT_INVALID_DATA;
   }
   for (uint32_t s = 0; s < n_streams; ++s)

@@ -125,7 +125,9 @@ __global__ void __launch_bounds__(GT, 1)
     const uint2* base = a.views ? a.nodes + a.views[s].x : a.nodes + (size_t)s * a.stride;
     uint2* nodes_out = a.nodes_out ? a.nodes_out + (size_t)s * a.stride : nullptr;
 
-    if (n > a.stride || n > ws.max_nodes) {  // caller error: report, touch nothing
+    // caller error (a count above the stride or the context's limit, a view that runs past the node buffer):
+    // report, touch nothing
+    if (n > a.stride || n > ws.max_nodes || (a.views && (unsigned long long)a.views[s].x + n > a.nodes_total)) {
       if (tid == 0) {
         if (a.status) a.status[s] = 0x80008000u;  // SL_RESULT_INVALID_DATA
         if (a.path) a.path[s] = 1u;

@@ -361,8 +361,11 @@ __global__ void __launch_bounds__(TS, POST ? 2 : (EMIT ? 4 : (MODE == 0 ? 5 : 1)
   uint32_t parity = 0;
 
   for (uint32_t s = blockIdx.x; s < a.n_scans; s += gridDim.x) {
-    const uint32_t n = a.views ? a.views[s].y : a.counts[s];
-    if (n > a.stride || n > p.max_nodes) {  // caller error: report, touch nothing
+    const uint2 view = a.views ? a.views[s] : make_uint2(0u, a.counts[s]);  // {first, count}
+    const uint32_t n = view.y;
+    // caller error (a count above the stride or the context's limit, a view that runs past the node buffer):
+    // report, touch nothing
+    if (n > a.stride || n > p.max_nodes || (a.views && (unsigned long long)view.x + n > a.nodes_total)) {
       if (tid == 0) {
         if (a.status) a.status[s] = 0x80008000u;  // SL_RESULT_INVALID_DATA
         if (a.path) a.path[s] = 0u;
@@ -380,7 +383,7 @@ __global__ void __launch_bounds__(TS, POST ? 2 : (EMIT ? 4 : (MODE == 0 ? 5 : 1)
       }
       continue;
     }
-    const uint2* base = a.views ? a.nodes + a.views[s].x : a.nodes + (size_t)s * a.stride;
+    const uint2* base = a.views ? a.nodes + view.x : a.nodes + (size_t)s * a.stride;
 
     // ---- stage the revolution (every thread is past the previous scan: its last barrier) -----------
     // Bulk copies move whole 16-byte units from 16-byte aligned addresses.  A batch scan starts aligned (even
@@ -391,7 +394,7 @@ __global__ void __launch_bounds__(TS, POST ? 2 : (EMIT ? 4 : (MODE == 0 ? 5 : 1)
     bool bulk = p.use_tma != 0;
     if (a.views) {
       shift = (uint32_t)((reinterpret_cast<uintptr_t>(base) >> 3) & 1u);
-      const unsigned long long first = a.views[s].x;
+      const unsigned long long first = view.x;
       bulk = bulk && (first - shift + ((n + shift + 1u) & ~1u) <= a.nodes_total);
     }
     const uint2* const tile = tile0 + shift;
